@@ -2,6 +2,7 @@
 """Benchmark of the MetaMorph hot path (contract: task statement + BASELINE.json).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (default N=1)
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs as DIR/*.npy
     python bench.py --impl reference --gpus N ...             # the reference's own code on the host cores (oracle/_ref)
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
@@ -44,7 +45,12 @@ def parse():
     ap.add_argument("--no-fused-allgather", action="store_true", help="A/B only: NCCL all-gather instead of the AdamW kernel's own broadcast")
     ap.add_argument("--extra-configs", default="auto", choices=["auto", "on", "off"],
                     help="BASELINE configs 3 (batch 8/GPU) and 5 (T=8192, 8 frames) as extra keys; auto = at 8 GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -316,6 +322,34 @@ def preprocess_bench(dev, peaks, n_images=16, h=480, w=640, iters=20):
             "cpu_baseline": cpu}
 
 
+DUMP_PARAM_SAMPLES = 4096      # per trainable tensor: ~200 tensors at 32 layers x 4096 x 4 B, a few MB
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, step_out, model):
+    """What the last timed step computed, as .npy files that two builds can be compared on: every value
+    TrainEngine.step returned (float64), and the trainable parameters it updated, as a fixed, seeded sample of
+    DUMP_PARAM_SAMPLES elements per tensor in named_parameters() order (float32; the full 8 B weights are 16 GB)."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for k, v in step_out.items():
+        arrays[k] = np.asarray(v.detach().cpu().double().numpy() if torch.is_tensor(v) else v, dtype=np.float64)
+    g = torch.Generator().manual_seed(0)
+    sample = []
+    for _, p in model.named_parameters():
+        if not p.requires_grad:
+            continue
+        idx = torch.randint(0, p.numel(), (min(DUMP_PARAM_SAMPLES, p.numel()),), generator=g)
+        sample.append(p.detach().reshape(-1)[idx.to(p.device)].float().cpu())
+    arrays["updated_params_sample"] = torch.cat(sample).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs: {total} bytes > {DUMP_MAX_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def run_reference_impl(args):
     """`--impl reference`: the reference's own CPU implementation of the path on the host cores, same metric/config.
     Every step is one bounded sample (see oracle/ref_bench.py); rank 0 alone runs it."""
@@ -425,7 +459,7 @@ def main():
             ops.GEMM_PROFILE = []
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        last = None
+        last = out = None
         for _ in range(steps):
             out = engine.step(batch)
             if read_loss:
@@ -442,15 +476,17 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t)
-        return ms, launches, prof, float(last)
+        return ms, launches, prof, float(last), out
 
     for _ in range(args.warmup):
         engine.step(dev_batch)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms, launches, prof, loss_val = timed(dev_batch, args.steps, read_loss=False, profile_gemm=True)
+    ms, launches, prof, loss_val, step_out = timed(dev_batch, args.steps, read_loss=False, profile_gemm=True)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_out, model)    # before the e2e steps below update the weights again
     tokens_per_step = world * B * T
     value = tokens_per_step * args.steps / (ms / 1e3)
 
@@ -485,7 +521,7 @@ def main():
 
     e2e = None
     if not args.no_e2e:
-        ms2, _, _, _ = timed(host_batch, args.steps, read_loss=True)
+        ms2, _, _, _, _ = timed(host_batch, args.steps, read_loss=True)
         h2d = host_batch["images"].numel() * 2 + (host_batch["input_ids"].numel() * 4 * 3)
         e2e = {"value": tokens_per_step * args.steps / (ms2 / 1e3), "unit": UNIT, "ms_per_step": ms2 / args.steps,
                "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": 4,
@@ -521,7 +557,7 @@ def main():
                 db["images"] = hb["images"].to(dev)
                 for _ in range(2):
                     engine.step(db)
-                ms_x, _, _, loss_x = timed(db, 3, read_loss=False)
+                ms_x, _, _, loss_x, _ = timed(db, 3, read_loss=False)
                 fl = train_flops_per_step(b_x, t_x, b_x * imgs_x, L=args.layers)
                 extra[key] = {"value": world * b_x * t_x * 3 / (ms_x / 1e3), "unit": UNIT, "ms_per_step": ms_x / 3,
                               "batch_per_gpu": b_x, "global_batch": world * b_x, "seq_len": t_x, "images_per_sample": imgs_x,
